@@ -250,10 +250,29 @@ def e2e_mi_render(workload, steps, device):
         return {"error": f"{type(e).__name__}: {str(e)[:160]}", "output_tail": tail}
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """Write every array as <out_dir>/<name>.npy in float32. When all of them together exceed DUMP_LIMIT_BYTES, an array
+    larger than its even share of the limit is replaced by a fixed sample of its rows along the first two axes (pixels
+    of an image): seed 0, sorted, so two runs with the same arguments sample the same pixels."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {k: np.asarray(v, np.float32) for k, v in arrays.items()}
+    share = DUMP_LIMIT_BYTES // max(1, len(arrays))
+    total = sum(a.nbytes for a in arrays.values())
+    for name, a in arrays.items():
+        if total > DUMP_LIMIT_BYTES and a.nbytes > share and a.ndim >= 2:
+            rows = a.reshape((a.shape[0] * a.shape[1],) + a.shape[2:])
+            n = max(1, share // (rows.nbytes // rows.shape[0]))
+            a = rows[np.sort(np.random.default_rng(0).choice(rows.shape[0], n, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
+    ap.add_argument("--steps", type=int, default=5, help="timed steps of every timed loop (device render, e2e, PRB gradient step)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--workload", default=DEFAULT_WORKLOAD, choices=sorted(WORKLOADS))
@@ -262,7 +281,14 @@ def main():
     ap.add_argument("--prb", action="store_true", help="(default on) also time the PRB gradient step (ms/grad-step)")
     ap.add_argument("--no-prb", action="store_true", help="skip the PRB gradient-step timing")
     ap.add_argument("--no-mi-render", action="store_true", help="skip the e2e leg through a live mi.render")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step of each timed loop returned as DIR/<name>.npy "
+                         "(float32; image, e2e_image, prb_image, prb_grad.<parameter>); inputs and seeds depend only on the arguments")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of --impl b200")
     if os.environ.get("B200PT_HANG_DUMP"):      # debugging aid: python stacks of all threads after N seconds
         import faulthandler
         faulthandler.dump_traceback_later(int(os.environ["B200PT_HANG_DUMP"]), exit=False)
@@ -322,11 +348,14 @@ def main():
     trace_ms = 0.0
     t0 = time.perf_counter(); ev0.record()
     for i in range(args.steps):
-        step_device(i)              # working set per step (wavefront state) >> L2, see DESIGN.md; nothing here waits for the device
+        image = step_device(i)      # working set per step (wavefront state) >> L2, see DESIGN.md; nothing here waits for the device
     ev1.record()
     sync_all()
     wall = time.perf_counter() - t0
     own_ms = ev0.elapsed_time(ev1)
+    outputs = {}
+    if args.dump_outputs:
+        outputs["image"] = image.cpu().numpy()     # the buffer is overwritten by the next render
     clk = clocks.stop()
     dev_ms = max_over_ranks(own_ms)
     ms_per_step = dev_ms / args.steps
@@ -393,6 +422,8 @@ def main():
         host_ms.append((time.perf_counter() - t_s) * 1e3)
     sync_all()
     e2e_s = max_over_ranks((time.perf_counter() - t1) / args.steps)
+    if args.dump_outputs:
+        outputs["e2e_image"] = np.array(img)
     e2e = {"value": samples_per_step / e2e_s / 1e6, "unit": "Msamples/s", "h2d_bytes_per_step": h2d,
            "d2h_bytes_per_step": img_bytes, "checksum": float(np.asarray(img).mean()),
            "per_step_ms": [round(x, 3) for x in host_ms],      # rank 0: wall time of every timed host step (an outlier shows here)
@@ -405,7 +436,7 @@ def main():
         scene_p, _ = build_scene(args.workload, textured_wall=True)      # configs[2]: wall albedo texture is the parameter
         gi = torch.full((h, w, 3), 1.0 / (h * w * 3), device=dev)
         spp_g = 64 * n_gpus if args.scaling == "weak" else 64
-        n_grad = max(3, args.steps // 2)
+        n_grad = args.steps
         for i in range(2):
             mbd.render_distributed(scene_p, pint, seed=50 + i, spp=spp_g, device=local)
             mbd.render_backward_distributed(scene_p, gi, pint, seed=150 + i, spp=spp_g, device=local)
@@ -413,11 +444,14 @@ def main():
         pe0, pe1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         pe0.record()
         for i in range(n_grad):
-            mbd.render_distributed(scene_p, pint, seed=i, spp=spp_g, device=local)
-            mbd.render_backward_distributed(scene_p, gi, pint, seed=100 + i, spp=spp_g, device=local)
+            prb_image = mbd.render_distributed(scene_p, pint, seed=i, spp=spp_g, device=local)
+            grads = mbd.render_backward_distributed(scene_p, gi, pint, seed=100 + i, spp=spp_g, device=local)
         pe1.record()
         sync_all()
         tp = max_over_ranks(pe0.elapsed_time(pe1))
+        if args.dump_outputs:
+            outputs["prb_image"] = prb_image.cpu().numpy()
+            outputs.update({f"prb_grad.{k}": v for k, v in grads.items()})
         pst = device_scene(scene_p, local).stats()
         n_params = int(sum(t.size for t in scene_p.textures if t.differentiable))
         # bytes of path state the gradient step streams (DESIGN.md section 5): primal pass + adjoint's own primal pass at
@@ -429,8 +463,10 @@ def main():
 
     mi_e2e = None
     if rank == 0 and world == 1 and not args.no_mi_render:
-        mi_e2e = e2e_mi_render(args.workload, min(args.steps, 5), local)
+        mi_e2e = e2e_mi_render(args.workload, args.steps, local)
 
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, outputs)
     if rank == 0:
         peaks = {}
         try:

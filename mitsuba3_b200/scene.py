@@ -827,13 +827,15 @@ def matpreview_like(n_theta: int = 256, n_phi: int = 512, env_res=(1024, 512)) -
 
 def matpreview_scene(path: str | None = None) -> dict:
     """BASELINE.json configs[3]: the reference's own asset resources/data/scenes/matpreview, from the arrays that
-    tests/golden/gen_matpreview.py extracted with the unmodified reference (three meshes as loaded, envmap.exr as linear
-    float32 RGB, envmap / sensor transforms). `bsdf-matpreview` is the principled model of SURVEY.md 8(d)
+    tests/golden/gen_matpreview.py extracted with the unmodified reference (three meshes as loaded, envmap / sensor
+    transforms; envmap.exr as linear float32 RGB in matpreview_envmap.npz beside `path`, a file of its own so that
+    neither exceeds 1 MB). `bsdf-matpreview` is the principled model of SURVEY.md 8(d)
     (base_color .94/.271/.361, roughness .3, metallic 0, specular .5); everything else follows matpreview.xml."""
     import os
     if path is None:
         path = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests", "golden", "matpreview_scene.npz")
     z = np.load(path, allow_pickle=False)
+    envmap = np.load(os.path.join(os.path.dirname(path), "matpreview_envmap.npz"), allow_pickle=False)["envmap"]
 
     def mesh(sid, bsdf):
         m = {"type": "mesh", "positions": z[f"{sid}|positions"], "texcoords": z[f"{sid}|texcoords"], "faces": z[f"{sid}|faces"], "bsdf": {"type": "ref", "id": bsdf}}
@@ -847,7 +849,7 @@ def matpreview_scene(path: str | None = None) -> dict:
                    "far_clip": float(z["sensor_clip"][1]), "to_world": Transform4f(z["sensor_to_world"]),
                    "sampler": {"type": "independent", "sample_count": 64},
                    "film": {"type": "hdrfilm", "width": 683, "height": 512, "pixel_format": "rgb", "rfilter": {"type": "gaussian"}}},
-        "emitter-envmap": {"type": "envmap", "data": z["envmap"], "scale": float(np.asarray(z["envmap_scale"]).reshape(-1)[0]), "to_world": Transform4f(z["envmap_to_world"])},
+        "emitter-envmap": {"type": "envmap", "data": envmap, "scale": float(np.asarray(z["envmap_scale"]).reshape(-1)[0]), "to_world": Transform4f(z["envmap_to_world"])},
         "bsdf-diffuse": {"type": "diffuse", "reflectance": {"type": "rgb", "value": [0.18, 0.18, 0.18]}},
         "bsdf-plane": {"type": "diffuse", "reflectance": {"type": "checkerboard", "color0": {"type": "rgb", "value": [0.4, 0.4, 0.4]},
                                                           "color1": {"type": "rgb", "value": [0.2, 0.2, 0.2]}, "to_uv": [[8, 0, 0], [0, 8, 0], [0, 0, 1]]}},

@@ -13,6 +13,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 def load_matpreview(mi, width, height, spp, max_depth=8, integrator="path"):
     import drjit as dr
     z = np.load(os.path.join(ROOT, "tests", "golden", "matpreview_scene.npz"), allow_pickle=False)
+    envmap = np.load(os.path.join(ROOT, "tests", "golden", "matpreview_envmap.npz"), allow_pickle=False)["envmap"]
     tmp = tempfile.mkdtemp(prefix="matpreview_")
 
     def ply(sid):
@@ -31,7 +32,7 @@ def load_matpreview(mi, width, height, spp, max_depth=8, integrator="path"):
                    "far_clip": float(z["sensor_clip"][1]), "to_world": T4(z["sensor_to_world"].tolist()),
                    "sampler": {"type": "independent", "sample_count": spp},
                    "film": {"type": "hdrfilm", "width": width, "height": height, "pixel_format": "rgb", "rfilter": {"type": "gaussian"}}},
-        "emitter-envmap": {"type": "envmap", "bitmap": mi.Bitmap(z["envmap"]), "scale": float(z["envmap_scale"]), "to_world": T4(z["envmap_to_world"].tolist())},
+        "emitter-envmap": {"type": "envmap", "bitmap": mi.Bitmap(envmap), "scale": float(z["envmap_scale"]), "to_world": T4(z["envmap_to_world"].tolist())},
         "bsdf-diffuse": {"type": "diffuse", "reflectance": {"type": "rgb", "value": [0.18, 0.18, 0.18]}},
         "bsdf-plane": {"type": "diffuse", "reflectance": {"type": "checkerboard", "color0": {"type": "rgb", "value": [0.4, 0.4, 0.4]},
                                                           "color1": {"type": "rgb", "value": [0.2, 0.2, 0.2]}, "to_uv": mi.ScalarTransform3f().scale([8, 8])}},

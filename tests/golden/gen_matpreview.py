@@ -66,8 +66,11 @@ def main():
     out["sensor_fov"] = np.array([28.8415], np.float32)
     out["sensor_clip"] = np.array([params["camera.near_clip"], params["camera.far_clip"]], np.float32)
     print("envmap", out["envmap"].shape, out["envmap"].dtype, "x_fov", params["camera.x_fov"])
+    # the envmap goes to a file of its own: together with the meshes it would exceed 1 MB
+    np.savez_compressed(os.path.join(HERE, "matpreview_envmap.npz"), envmap=out.pop("envmap"))
     np.savez_compressed(os.path.join(HERE, "matpreview_scene.npz"), **out)
-    print("wrote matpreview_scene.npz", os.path.getsize(os.path.join(HERE, "matpreview_scene.npz")) / 1e6, "MB")
+    for f in ("matpreview_scene.npz", "matpreview_envmap.npz"):
+        print("wrote", f, os.path.getsize(os.path.join(HERE, f)) / 1e6, "MB")
     ren = {}
     for (res, spp, seed) in [(64, 16, 0), (96, 8, 3)]:
         sc = load(res, res, spp)

@@ -413,7 +413,7 @@ b200pt_status b200pt_scene_create(const b200pt_scene_desc *desc, int device, b20
     s->launch.smem_tables = (d.tables_bytes <= 12288 ? d.tables_bytes : 0) + (d.geom_bytes <= 20480 ? d.geom_bytes : 0);
     { const char *e = getenv("B200PT_TRACE_BLOCKS_PER_SM"); s->launch.grid = (int) s->n_sm * (e ? std::max(1, atoi(e)) : 5); }
     { const char *e = getenv("B200PT_REFILL_IDLE"); s->launch.refill_idle = e ? std::min(32, std::max(1, atoi(e))) : 8; }
-    {   // scenes of at most 32 leaves whose tree and triangles are staged whole: flat traversal (kernels.cu: traverse_flat)
+    {   // scenes of at most 32 leaves whose tree and triangles are staged whole: flat traversal (kernels.cu: k_trace_flat)
         uint32_t n_leaves = 0;
         for (const auto &nd : bvh.nodes) { if (nd.left < 0) n_leaves++; if (nd.right < 0) n_leaves++; }
         const char *e = getenv("B200PT_FLAT_TRAVERSAL");

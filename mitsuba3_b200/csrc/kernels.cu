@@ -147,7 +147,7 @@ PT_DEV bool box_hit(float lox, float loy, float loz, float hix, float hiy, float
     return tmin <= tmx * 1.0000004f;
 }
 
-// Slab test in fused form (flat traversal: 18+ boxes per ray, registers to spare): t = lo * inv - (o * inv), one FFMA per
+// Slab test in fused form (flat traversal, flat_phase: 18+ boxes per ray, registers to spare): t = lo * inv - (o * inv), one FFMA per
 // plane instead of a subtraction and a multiplication. The product o * inv is rounded once per ray, so a plane distance is off
 // by up to 2^-24 |o * inv| against the exact (lo - o) * inv; `slack` = 2^-22 max |o * inv| widens the interval test by more
 // than twice that. The boxes only cull -- a hit is only ever decided by the reference's Moeller-Trumbore arithmetic -- so a
@@ -161,15 +161,6 @@ PT_DEV RaySlabs make_slabs(float3 o, float3 d) {
     r.oi = V(o.x * r.inv.x, o.y * r.inv.y, o.z * r.inv.z);
     r.slack = fmaxf(fmaxf(fabsf(r.oi.x), fabsf(r.oi.y)), fabsf(r.oi.z)) * 2.3841858e-7f;
     return r;
-}
-PT_DEV bool box_hit(float lox, float loy, float loz, float hix, float hiy, float hiz, const RaySlabs &r, float tmax, float &tnear) {
-    float t0x = __fmaf_rn(lox, r.inv.x, -r.oi.x), t1x = __fmaf_rn(hix, r.inv.x, -r.oi.x);
-    float t0y = __fmaf_rn(loy, r.inv.y, -r.oi.y), t1y = __fmaf_rn(hiy, r.inv.y, -r.oi.y);
-    float t0z = __fmaf_rn(loz, r.inv.z, -r.oi.z), t1z = __fmaf_rn(hiz, r.inv.z, -r.oi.z);
-    float tmin = fmaxf(fmaxf(fminf(t0x, t1x), fminf(t0y, t1y)), fmaxf(fminf(t0z, t1z), 0.f));
-    float tmx = fminf(fminf(fmaxf(t0x, t1x), fmaxf(t0y, t1y)), fminf(fmaxf(t0z, t1z), tmax));
-    tnear = tmin;
-    return tmin <= __fmaf_rn(tmx, 1.0000004f, r.slack);
 }
 
 // Speculative while-while traversal (Aila & Laine, "Understanding the Efficiency of Ray
@@ -228,67 +219,53 @@ PT_DEV bool traverse(const TraceCtx &c, float3 o, float3 d, float maxt, Hit &hit
 }
 
 // ---------------------------------------------------------------------------
-// Flat traversal for scenes of at most FLAT_MAX_LEAVES leaves (the Cornell box: 36 triangles in 18+ leaves). In a closed
+// Flat traversal for scenes of at most FLAT_MAX_LEAVES leaves (the Cornell box: 36 triangles in 18 leaves). In a closed
 // room the top of a binary tree culls nothing -- every inner box near the root spans the room -- so a walk spends ~10
 // divergent node steps per ray before it reaches the two or three leaves that matter. Here every lane tests the boxes of
-// ALL leaves in the same order instead (one broadcast LDS pair and ~16 arithmetic instructions per leaf, 32 of 32 threads
-// active, no stack), keeps the hit boxes as a bit mask, and then runs the reference's Moeller-Trumbore on the candidate
-// leaves only: the nearest box first, the others re-tested against the shortened ray. Results are those of any other
+// ALL leaves in the same order instead (32 of 32 threads active, no stack), keeps the hit boxes as a bit mask, and then runs
+// the reference's Moeller-Trumbore on the candidate leaves only (k_trace_flat, flat_phase). Results are those of any other
 // traversal order: closest hit with ties resolved towards the smaller primitive index, any-hit a boolean.
 // ---------------------------------------------------------------------------
 constexpr uint32_t FLAT_MAX_LEAVES = 32;
+constexpr uint32_t FLAT_UNROLL = 3;                 // leaves per iteration of the box pass; the list is padded to a multiple
+constexpr uint32_t FLAT_LEAF_SLOTS = (FLAT_MAX_LEAVES + FLAT_UNROLL - 1) / FLAT_UNROLL * FLAT_UNROLL;
+constexpr uint32_t FLAT_MAX_TRIS = 256;
 
-// Leaf list from the staged nodes: every negative child of an inner node is a leaf; entry l = { (lo.xyz, hi.x), (hi.yz, leaf code, -) }.
-PT_DEV void build_leaf_list(const float4 *s_nodes, uint32_t n_nodes, float4 *s_leaf, uint32_t *s_nleaf) {
-    if (threadIdx.x == 0) *s_nleaf = 0;
+// Leaf boxes ordered by direction octant: box[l][0][oct] holds the near-plane coordinates of leaf l for a ray whose inv
+// has the sign bits oct (bit 0: x, 1: y, 2: z; a set bit makes `hi` the near plane of that axis), box[l][1][oct] the far
+// ones. For inv >= 0, fma(lo, inv, -oi) <= fma(hi, inv, -oi) because rounding is monotone, and the reverse for inv < 0, so
+// the near/far values are exactly what fminf / fmaxf of the two plane distances would pick: the box pass needs no per-axis
+// min/max. The 8 copies of one leaf's near (far) planes fill one 128-byte line, so a warp's loads of one leaf never
+// conflict, whatever mix of octants its rays hold. `.w` of the near copies is the leaf code (bvh.h), of the far copies
+// the leaf index. Slots n .. n_pad-1 are empty boxes (lo = +inf, hi = -inf: the near distance is +inf, the far -inf,
+// never a hit).
+struct FlatLeaves { float4 box[FLAT_LEAF_SLOTS][2][8]; uint32_t n; };
+
+PT_DEV void put_flat_leaf(FlatLeaves &L, uint32_t k, float3 lo, float3 hi, uint32_t code) {
+    for (uint32_t oc = 0; oc < 8; ++oc) {
+        const bool sx = oc & 1u, sy = oc & 2u, sz = oc & 4u;
+        L.box[k][0][oc] = make_float4(sx ? hi.x : lo.x, sy ? hi.y : lo.y, sz ? hi.z : lo.z, __uint_as_float(code));
+        L.box[k][1][oc] = make_float4(sx ? lo.x : hi.x, sy ? lo.y : hi.y, sz ? lo.z : hi.z, __uint_as_float(k));
+    }
+}
+
+// Leaf list from the staged nodes (every negative child of an inner node is a leaf), padded to a multiple of FLAT_UNROLL,
+// and the map primitive id -> staged triangle. Returns the padded leaf count.
+PT_DEV uint32_t build_leaf_list(const float4 *s_nodes, uint32_t n_nodes, const float4 *s_tris, uint32_t n_tris, FlatLeaves &L, uint8_t *s_primmap) {
+    if (threadIdx.x == 0) L.n = 0;
     __syncthreads();
     for (uint32_t node = threadIdx.x; node < n_nodes; node += blockDim.x) {
         float4 n0 = s_nodes[4 * node], n1 = s_nodes[4 * node + 1], n2 = s_nodes[4 * node + 2], n3 = s_nodes[4 * node + 3];
         int32_t cl = __float_as_int(n3.x), cr = __float_as_int(n3.y);
-        if (cl < 0) { uint32_t k = atomicAdd(s_nleaf, 1u); if (k < FLAT_MAX_LEAVES) { s_leaf[2 * k] = make_float4(n0.x, n0.y, n0.z, n0.w); s_leaf[2 * k + 1] = make_float4(n1.x, n1.y, __int_as_float(~cl), 0.f); } }
-        if (cr < 0) { uint32_t k = atomicAdd(s_nleaf, 1u); if (k < FLAT_MAX_LEAVES) { s_leaf[2 * k] = make_float4(n1.z, n1.w, n2.x, n2.y); s_leaf[2 * k + 1] = make_float4(n2.z, n2.w, __int_as_float(~cr), 0.f); } }
+        if (cl < 0) { uint32_t k = atomicAdd(&L.n, 1u); if (k < FLAT_MAX_LEAVES) put_flat_leaf(L, k, V(n0.x, n0.y, n0.z), V(n0.w, n1.x, n1.y), (uint32_t) ~cl); }
+        if (cr < 0) { uint32_t k = atomicAdd(&L.n, 1u); if (k < FLAT_MAX_LEAVES) put_flat_leaf(L, k, V(n1.z, n1.w, n2.x), V(n2.y, n2.z, n2.w), (uint32_t) ~cr); }
     }
+    for (uint32_t i = threadIdx.x; i < n_tris; i += blockDim.x) s_primmap[__float_as_uint(s_tris[3 * i].w) & (FLAT_MAX_TRIS - 1u)] = (uint8_t) i;
     __syncthreads();
-}
-
-template <bool ANY>
-PT_DEV bool traverse_flat(const float4 *s_leaf, uint32_t n_leaves, const float4 *s_tris, float3 o, float3 d, float maxt, Hit &hit) {
-    hit.t = PT_INF; hit.u = hit.v = 0.f; hit.prim = 0xffffffffu;
-    const RaySlabs rs = make_slabs(o, d);
-    uint32_t mask = 0; float best_tn = PT_INF; uint32_t best = 0;
-#pragma unroll 3
-    for (uint32_t l = 0; l < n_leaves; ++l) {
-        float4 a = s_leaf[2 * l], b = s_leaf[2 * l + 1];
-        float tn;
-        if (box_hit(a.x, a.y, a.z, a.w, b.x, b.y, rs, maxt, tn)) {
-            mask |= 1u << l;
-            if (!ANY && tn < best_tn) { best_tn = tn; best = l; }
-        }
-    }
-    bool any = false;
-    bool first = !ANY && mask != 0;           // closest hit: the nearest box goes first
-    while (mask) {
-        uint32_t l;
-        if (first) l = best; else l = (uint32_t) __ffs((int) mask) - 1u;
-        mask &= ~(1u << l);
-        float4 b = s_leaf[2 * l + 1];
-        if (!ANY && any) {                     // the ray has been shortened since the box pass
-            float4 a = s_leaf[2 * l]; float tn;
-            if (!box_hit(a.x, a.y, a.z, a.w, b.x, b.y, rs, maxt, tn)) continue;
-        }
-        first = false;
-        uint32_t enc = __float_as_uint(b.z), t0 = enc >> 3, count = (enc & 7u) + 1u;
-        for (uint32_t i = t0; i < t0 + count; ++i) {
-            float4 ta = s_tris[3 * i], tb = s_tris[3 * i + 1], te = s_tris[3 * i + 2];
-            float t, u, v;
-            if (moeller_trumbore(o, d, maxt, V(ta.x, ta.y, ta.z), V(tb.x, tb.y, tb.z), V(te.x, te.y, te.z), t, u, v)) {
-                if (ANY) return true;
-                uint32_t prim = __float_as_uint(ta.w);
-                if (t < hit.t || (t == hit.t && prim < hit.prim)) { hit.t = t; hit.u = u; hit.v = v; hit.prim = prim; maxt = t; any = true; }
-            }
-        }
-    }
-    return any;
+    const uint32_t n = min(L.n, FLAT_MAX_LEAVES), n_pad = (n + FLAT_UNROLL - 1) / FLAT_UNROLL * FLAT_UNROLL;
+    if (threadIdx.x >= n && threadIdx.x < n_pad) put_flat_leaf(L, threadIdx.x, V(PT_INF, PT_INF, PT_INF), V(-PT_INF, -PT_INF, -PT_INF), 0u);
+    __syncthreads();
+    return n_pad;
 }
 
 // ---------------------------------------------------------------------------
@@ -329,9 +306,10 @@ __global__ void __launch_bounds__(BLOCK) k_generate(DevScene sc, RenderCfg cfg, 
 //   3. finished lanes write their radiance to lane_result (consumed by k_splat)
 // ---------------------------------------------------------------------------
 // ---------------------------------------------------------------------------
-// k_trace_flat -- the traversal kernel of scenes with at most FLAT_MAX_LEAVES leaves (see traverse_flat). Same work per
+// k_trace_flat -- the traversal kernel of scenes with at most FLAT_MAX_LEAVES leaves (see FlatLeaves). Same work per
 // slot as k_trace, organised in warp-wide phases so that the exact triangle tests are shared by the whole warp:
-//   box pass    every lane tests its own ray against all leaf boxes (32 of 32 threads, registers only) -> candidate mask
+//   box pass    every lane tests its own ray against all leaf boxes (32 of 32 threads, the octant's near / far planes:
+//               2 LDS.128, 6 FFMA, 4 FMNMX, 1 FFMA, 1 FSETP and one predicated LOP3 per leaf) -> candidate mask
 //   pair list   the (ray, leaf) candidates of the 32 rays are written to one list in shared memory (warp prefix sum)
 //   test rounds lane j tests pairs j, j + 32, ...: the reference's Moeller-Trumbore on another lane's ray (the rays sit in
 //               shared memory); closest hit = 64-bit atomicMin on (t bits, primitive id) per ray -- the same minimum and
@@ -341,7 +319,6 @@ __global__ void __launch_bounds__(BLOCK) k_generate(DevScene sc, RenderCfg cfg, 
 // of the kernel's instructions; the rounds run them at ~30 of 32.
 // ---------------------------------------------------------------------------
 constexpr uint32_t FLAT_PAIR_CAP = 32 * FLAT_MAX_LEAVES;      // candidate (ray, leaf) pairs of one warp and phase: every pair fits
-constexpr uint32_t FLAT_MAX_TRIS = 256;
 
 struct FlatWarp {          // per-warp scratch in shared memory
     float4 ray[64];                        // (o, maxt), (d, -) of the 32 rays of the phase
@@ -352,52 +329,97 @@ struct FlatWarp {          // per-warp scratch in shared memory
 
 // One phase for the 32 rays of a warp; called by all 32 lanes at a converged point. ANY: returns "occluded"; otherwise the
 // closest hit in `hit`.
+// Closest hit tests the lane's nearest candidate leaf (smallest box entry distance) on the lane itself first and hands
+// to the shared rounds only the candidates whose entry distance is at most lim = t * (1 + 2^-10) + slack, t the hit found
+// there. A leaf beyond lim holds no hit at t or closer: the box pass culls against maxt with a margin of 4e-7 relative
+// plus the same slack, and 2^-10 is more than 2000 times that. Hits at an equal t in a neighbouring leaf (shared edges,
+// the corners of a room) stay inside the margin and meet the own hit in the same (t bits, primitive) minimum.
 template <bool ANY>
-PT_DEV bool flat_phase(FlatWarp &w, const float4 *s_leaf, uint32_t n_leaves, const float4 *s_tris, const uint8_t *s_primmap,
+PT_DEV bool flat_phase(FlatWarp &w, const FlatLeaves &L, uint32_t n_pad, const float4 *s_tris, const uint8_t *s_primmap,
                        bool active, float3 o, float3 d, float maxt, Hit &hit) {
     const uint32_t lane_id = threadIdx.x & 31u;
     hit.t = PT_INF; hit.u = hit.v = 0.f; hit.prim = 0xffffffffu;
     uint32_t mask = 0;
+    unsigned long long own = ~0ull;            // closest hit in the nearest candidate leaf: (t bits << 32) | primitive id
+    float own_t = 0.f, own_u = 0.f, own_v = 0.f;
     if (active) {
         const RaySlabs rs = make_slabs(o, d);
-#pragma unroll 3
-        for (uint32_t l = 0; l < n_leaves; ++l) {
-            float4 a = s_leaf[2 * l], b = s_leaf[2 * l + 1];
-            float tn;
-            if (box_hit(a.x, a.y, a.z, a.w, b.x, b.y, rs, maxt, tn)) mask |= 1u << l;
-        }
-        w.ray[2 * lane_id] = make_float4(o.x, o.y, o.z, maxt); w.ray[2 * lane_id + 1] = make_float4(d.x, d.y, d.z, 0.f);
-    }
-    if (ANY) w.occ[lane_id] = 0u; else w.key[lane_id] = ~0ull;
-    // exclusive prefix sum of the candidate counts
-    const uint32_t cnt = (uint32_t) __popc(mask);
-    uint32_t incl = cnt;
+        const uint32_t oct = (__float_as_uint(rs.inv.x) >> 31) | (__float_as_uint(rs.inv.y) >> 31 << 1) | (__float_as_uint(rs.inv.z) >> 31 << 2);
+        const float4 *bx = &L.box[0][0][oct];
+        uint32_t nearest = ~0u;                // entry distance bits with the leaf index in the low 5 bits: the smallest wins
+#pragma unroll 1
+        for (uint32_t l = 0; l < n_pad; l += FLAT_UNROLL, bx += FLAT_UNROLL * 16) {
+            uint32_t g = 0;
 #pragma unroll
-    for (int of = 1; of < 32; of <<= 1) { uint32_t v = __shfl_up_sync(0xffffffffu, incl, of); if ((int) lane_id >= of) incl += v; }
-    const uint32_t total = __shfl_sync(0xffffffffu, incl, 31);
-    if (total == 0) return false;
-    {   // pair list: (ray << 8) | leaf
-        uint32_t k = incl - cnt, m = mask;
-        while (m) { uint32_t l = (uint32_t) __ffs((int) m) - 1u; m &= m - 1u; w.pairs[k++] = (uint16_t) ((lane_id << 8) | l); }
-    }
-    __syncwarp();
-    for (uint32_t p = lane_id; p < total; p += 32u) {
-        const uint32_t e = w.pairs[p], r = e >> 8, l = e & 255u;
-        const float4 ro = w.ray[2 * r], rd = w.ray[2 * r + 1];
-        const uint32_t enc = __float_as_uint(s_leaf[2 * l + 1].z), t0 = enc >> 3, count = (enc & 7u) + 1u;
-        for (uint32_t ti = t0; ti < t0 + count; ++ti) {
-            const float4 ta = s_tris[3 * ti], tb = s_tris[3 * ti + 1], te = s_tris[3 * ti + 2];
-            float t, u, v;
-            if (moeller_trumbore(V(ro.x, ro.y, ro.z), V(rd.x, rd.y, rd.z), ro.w, V(ta.x, ta.y, ta.z), V(tb.x, tb.y, tb.z), V(te.x, te.y, te.z), t, u, v)) {
-                if (ANY) w.occ[r] = 1u;
-                else atomicMin(&w.key[r], ((unsigned long long) __float_as_uint(t + 0.f) << 32) | __float_as_uint(ta.w));   // t >= 0: its bits order like its value; -0 -> +0
+            for (uint32_t j = 0; j < FLAT_UNROLL; ++j) {
+                // box_hit with the near / far plane of every axis known in advance: the same values, the same predicate
+                const float4 nr = bx[16 * j], fr = bx[16 * j + 8];
+                const float nx = __fmaf_rn(nr.x, rs.inv.x, -rs.oi.x), ny = __fmaf_rn(nr.y, rs.inv.y, -rs.oi.y), nz = __fmaf_rn(nr.z, rs.inv.z, -rs.oi.z);
+                const float fx = __fmaf_rn(fr.x, rs.inv.x, -rs.oi.x), fy = __fmaf_rn(fr.y, rs.inv.y, -rs.oi.y), fz = __fmaf_rn(fr.z, rs.inv.z, -rs.oi.z);
+                const float tmin = fmaxf(fmaxf(nx, ny), fmaxf(nz, 0.f)), tmx = fminf(fminf(fx, fy), fminf(fz, maxt));
+                if (tmin <= __fmaf_rn(tmx, 1.0000004f, rs.slack)) {
+                    g |= 1u << j;
+                    if (!ANY) nearest = min(nearest, (__float_as_uint(tmin) & 0x7fffffe0u) | __float_as_uint(fr.w));
+                }
+            }
+            mask |= g << l;
+        }
+        if (!ANY && mask) {
+            const uint32_t l0 = nearest & 31u, enc = __float_as_uint(L.box[l0][0][0].w), t0 = enc >> 3, count = (enc & 7u) + 1u;
+            mask &= ~(1u << l0);
+            for (uint32_t ti = t0; ti < t0 + count; ++ti) {
+                const float4 ta = s_tris[3 * ti], tb = s_tris[3 * ti + 1], te = s_tris[3 * ti + 2];
+                float t, u, v;
+                if (moeller_trumbore(o, d, maxt, V(ta.x, ta.y, ta.z), V(tb.x, tb.y, tb.z), V(te.x, te.y, te.z), t, u, v)) {
+                    const unsigned long long k = ((unsigned long long) __float_as_uint(t + 0.f) << 32) | __float_as_uint(ta.w);
+                    if (k < own) { own = k; own_t = t; own_u = u; own_v = v; }
+                }
+            }
+            if (own != ~0ull) {
+                const float lim = __fmaf_rn(__uint_as_float((uint32_t) (own >> 32)), 1.0009765625f, rs.slack);
+                for (uint32_t m = mask; m; m &= m - 1u) {
+                    const uint32_t l = (uint32_t) __ffs((int) m) - 1u;
+                    const float4 nr = L.box[l][0][oct];
+                    const float nx = __fmaf_rn(nr.x, rs.inv.x, -rs.oi.x), ny = __fmaf_rn(nr.y, rs.inv.y, -rs.oi.y), nz = __fmaf_rn(nr.z, rs.inv.z, -rs.oi.z);
+                    if (fmaxf(fmaxf(nx, ny), fmaxf(nz, 0.f)) > lim) mask &= ~(1u << l);
+                }
             }
         }
     }
-    __syncwarp();
-    if (ANY) return active && w.occ[lane_id] != 0u;
-    const unsigned long long key = w.key[lane_id];
-    if (!active || key == ~0ull) return false;
+    unsigned long long key = own;
+    if (__any_sync(0xffffffffu, mask != 0u)) {
+        if (mask) { w.ray[2 * lane_id] = make_float4(o.x, o.y, o.z, maxt); w.ray[2 * lane_id + 1] = make_float4(d.x, d.y, d.z, 0.f); }
+        if (ANY) w.occ[lane_id] = 0u; else w.key[lane_id] = own;
+        // exclusive prefix sum of the candidate counts
+        const uint32_t cnt = (uint32_t) __popc(mask);
+        uint32_t incl = cnt;
+#pragma unroll
+        for (int of = 1; of < 32; of <<= 1) { uint32_t v = __shfl_up_sync(0xffffffffu, incl, of); if ((int) lane_id >= of) incl += v; }
+        const uint32_t total = __shfl_sync(0xffffffffu, incl, 31);
+        {   // pair list: (ray << 8) | leaf
+            uint32_t k = incl - cnt, m = mask;
+            while (m) { uint32_t l = (uint32_t) __ffs((int) m) - 1u; m &= m - 1u; w.pairs[k++] = (uint16_t) ((lane_id << 8) | l); }
+        }
+        __syncwarp();
+        for (uint32_t p = lane_id; p < total; p += 32u) {
+            const uint32_t e = w.pairs[p], r = e >> 8, l = e & 255u;
+            const float4 ro = w.ray[2 * r], rd = w.ray[2 * r + 1];
+            const uint32_t enc = __float_as_uint(L.box[l][0][0].w), t0 = enc >> 3, count = (enc & 7u) + 1u;
+            for (uint32_t ti = t0; ti < t0 + count; ++ti) {
+                const float4 ta = s_tris[3 * ti], tb = s_tris[3 * ti + 1], te = s_tris[3 * ti + 2];
+                float t, u, v;
+                if (moeller_trumbore(V(ro.x, ro.y, ro.z), V(rd.x, rd.y, rd.z), ro.w, V(ta.x, ta.y, ta.z), V(tb.x, tb.y, tb.z), V(te.x, te.y, te.z), t, u, v)) {
+                    if (ANY) w.occ[r] = 1u;
+                    else atomicMin(&w.key[r], ((unsigned long long) __float_as_uint(t + 0.f) << 32) | __float_as_uint(ta.w));   // t >= 0: its bits order like its value; -0 -> +0
+                }
+            }
+        }
+        __syncwarp();
+        if (ANY) return active && w.occ[lane_id] != 0u;
+        key = w.key[lane_id];
+    }
+    if (ANY || !active || key == ~0ull) return false;
+    if (key == own) { hit.t = own_t; hit.u = own_u; hit.v = own_v; hit.prim = (uint32_t) key; return true; }
     const uint32_t ti = s_primmap[(uint32_t) key];
     const float4 ta = s_tris[3 * ti], tb = s_tris[3 * ti + 1], te = s_tris[3 * ti + 2];
     float t, u, v;
@@ -412,8 +434,7 @@ __global__ void __launch_bounds__(BLOCK, 4) k_trace_flat(const __grid_constant__
                                                          unsigned long long *__restrict__ stats, uint32_t n_smem_nodes, uint32_t n_smem_tris) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     __shared__ uint64_t bar;
-    __shared__ float4 s_leaf[2 * FLAT_MAX_LEAVES];
-    __shared__ uint32_t s_nleaf;
+    __shared__ FlatLeaves s_leaves;
     __shared__ uint8_t s_primmap[FLAT_MAX_TRIS];
     __shared__ FlatWarp s_warp[BLOCK / 32];
     DevScene sc = sc_in;
@@ -423,10 +444,7 @@ __global__ void __launch_bounds__(BLOCK, 4) k_trace_flat(const __grid_constant__
     __syncthreads();
     stage_bvh(sc, s_nodes, s_tris, n_smem_nodes, n_smem_tris, &bar);
     stage_tables(sc, smem_raw + ((n_smem_nodes * 64u + n_smem_tris * 48u + 127u) & ~127u), &bar, 1u);
-    build_leaf_list(s_nodes, n_smem_nodes, s_leaf, &s_nleaf);
-    for (uint32_t i = threadIdx.x; i < n_smem_tris; i += blockDim.x) s_primmap[__float_as_uint(s_tris[3 * i].w) & (FLAT_MAX_TRIS - 1u)] = (uint8_t) i;
-    __syncthreads();
-    const uint32_t n_leaves = min(s_nleaf, FLAT_MAX_LEAVES);
+    const uint32_t n_pad = build_leaf_list(s_nodes, n_smem_nodes, s_tris, n_smem_tris, s_leaves, s_primmap);
     FlatWarp &w = s_warp[threadIdx.x >> 5];
 
     const uint32_t n = FIRST ? cfg.chunk_lanes : *n_in;
@@ -445,7 +463,7 @@ __global__ void __launch_bounds__(BLOCK, 4) k_trace_flat(const __grid_constant__
             float4 so = make_float4(0.f, 0.f, 0.f, 0.f), sd = make_float4(0.f, 0.f, 1.f, 0.f);
             if (has_shadow) { so = cur.sh_o[i]; sd = cur.sh_d[i]; n_shadow++; }
             Hit hs;
-            const bool occluded = flat_phase<true>(w, s_leaf, n_leaves, s_tris, s_primmap, has_shadow, V(so.x, so.y, so.z), V(sd.x, sd.y, sd.z), so.w, hs);
+            const bool occluded = flat_phase<true>(w, s_leaves, n_pad, s_tris, s_primmap, has_shadow, V(so.x, so.y, so.z), V(sd.x, sd.y, sd.z), so.w, hs);
             if (has_shadow && !occluded) {
                 if (cur.vis) { uint32_t bit = (flags & PF_DEPTH_MASK) - 1u; if (bit < 32u) cur.vis[cur.rng[i].w] |= 1u << bit; }
                 float2 c = cur.sh_c[i];
@@ -463,7 +481,7 @@ __global__ void __launch_bounds__(BLOCK, 4) k_trace_flat(const __grid_constant__
             float3 o = V(0.f, 0.f, 0.f), d = V(0.f, 0.f, 1.f); float maxt = 0.f;
             if (alive) { float4 ro = cur.ray_o[i], rd = cur.ray_d[i]; o = V(ro.x, ro.y, ro.z); d = V(rd.x, rd.y, rd.z); maxt = ro.w; n_closest++; }
             Hit h;
-            bool found = flat_phase<false>(w, s_leaf, n_leaves, s_tris, s_primmap, alive, o, d, maxt, h);
+            bool found = flat_phase<false>(w, s_leaves, n_pad, s_tris, s_primmap, alive, o, d, maxt, h);
             if (FIRST && cfg.hide_emitters) {
                 // skip_area_emitters (integrator.cpp:96-123): continue through directly visible emitters
                 bool again = alive && found && sc.shapes[sc.prim_verts[h.prim].w].emitter >= 0;
@@ -476,7 +494,7 @@ __global__ void __launch_bounds__(BLOCK, 4) k_trace_flat(const __grid_constant__
                     }
                     __syncwarp();
                     Hit h2;
-                    bool f2 = flat_phase<false>(w, s_leaf, n_leaves, s_tris, s_primmap, again, o, d, maxt, h2);
+                    bool f2 = flat_phase<false>(w, s_leaves, n_pad, s_tris, s_primmap, again, o, d, maxt, h2);
                     if (again) { found = f2; h = h2; again = found && sc.shapes[sc.prim_verts[h.prim].w].emitter >= 0; }
                     __syncwarp();
                 }
@@ -1303,20 +1321,37 @@ __global__ void __launch_bounds__(BLOCK) k_ray_query(DevScene sc, uint32_t n, co
     __syncthreads();
     stage_bvh(sc, s_nodes, s_tris, n_smem_nodes, n_smem_tris, &bar);
     TraceCtx ctx = { s_nodes, s_tris, sc.nodes, sc.tris, n_smem_nodes, n_smem_tris };
-    __shared__ float4 s_leaf[2 * FLAT_MAX_LEAVES];
-    __shared__ uint32_t s_nleaf;
-    if (flat) build_leaf_list(s_nodes, n_smem_nodes, s_leaf, &s_nleaf);     // the traversal the render kernels use for this scene
-    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
-        const float *r = rays + 7 * (size_t) i;
-        Hit h;
-        bool found = flat ? traverse_flat<ANY>(s_leaf, min(s_nleaf, FLAT_MAX_LEAVES), s_tris, V(r[0], r[1], r[2]), V(r[3], r[4], r[5]), r[6], h)
-                          : traverse<ANY, false>(ctx, V(r[0], r[1], r[2]), V(r[3], r[4], r[5]), r[6], h);
-        if (ANY) { occ_out[i] = found ? 1 : 0; continue; }
+    auto put = [&](uint32_t i, bool found, const Hit &h) {
+        if (ANY) { occ_out[i] = found ? 1 : 0; return; }
         t_out[i] = found ? h.t : PT_INF; uv_out[2 * i] = found ? h.u : 0.f; uv_out[2 * i + 1] = found ? h.v : 0.f;
         if (found) {
             uint4 pv = sc.prim_verts[h.prim];
             shape_out[i] = (int32_t) pv.w; prim_out[i] = h.prim - sc.shapes[pv.w].first_prim;
         } else { shape_out[i] = -1; prim_out[i] = 0; }
+    };
+    if (flat) {         // the traversal the render kernels use for this scene, in the same warp-uniform loop as k_trace_flat
+        __shared__ FlatLeaves s_leaves;
+        __shared__ uint8_t s_primmap[FLAT_MAX_TRIS];
+        __shared__ FlatWarp s_warp[BLOCK / 32];
+        const uint32_t n_pad = build_leaf_list(s_nodes, n_smem_nodes, s_tris, n_smem_tris, s_leaves, s_primmap);
+        FlatWarp &w = s_warp[threadIdx.x >> 5];
+        for (uint32_t base = blockIdx.x * blockDim.x + (threadIdx.x & ~31u); base < n; base += gridDim.x * blockDim.x) {
+            const uint32_t i = base + (threadIdx.x & 31u);
+            const bool valid = i < n;
+            float3 o = V(0.f, 0.f, 0.f), d = V(0.f, 0.f, 1.f); float maxt = 0.f;
+            if (valid) { const float *r = rays + 7 * (size_t) i; o = V(r[0], r[1], r[2]); d = V(r[3], r[4], r[5]); maxt = r[6]; }
+            Hit h;
+            const bool found = flat_phase<ANY>(w, s_leaves, n_pad, s_tris, s_primmap, valid, o, d, maxt, h);
+            if (valid) put(i, found, h);
+            __syncwarp();
+        }
+        return;
+    }
+    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+        const float *r = rays + 7 * (size_t) i;
+        Hit h;
+        const bool found = traverse<ANY, false>(ctx, V(r[0], r[1], r[2]), V(r[3], r[4], r[5]), r[6], h);
+        put(i, found, h);
     }
 }
 
@@ -1351,7 +1386,7 @@ void launch_generate(const DevScene &sc, const RenderCfg &cfg, const uint32_t *p
 void launch_trace(const DevScene &sc, const RenderCfg &cfg, PathBuf cur, float4 *hit, const uint32_t *n_in, Queues q, uint32_t *qcounts,
                   float4 *lane_result, unsigned long long *stats, bool first, const Launch &L, cudaStream_t st) {
     bool all = L.n_smem_nodes == sc.n_nodes && L.n_smem_tris == sc.n_tris;
-    if (L.flat) {       // <= FLAT_MAX_LEAVES leaves: every lane tests every leaf box, no tree walk (see traverse_flat)
+    if (L.flat) {       // <= FLAT_MAX_LEAVES leaves: every lane tests every leaf box, no tree walk (see k_trace_flat)
         int grid = L.grid_flat;
         if (first) k_trace_flat<true><<<grid, BLOCK, L.smem_trace + L.smem_tables, st>>>(sc, cfg, cur, hit, n_in, q, qcounts, lane_result, stats, L.n_smem_nodes, L.n_smem_tris);
         else k_trace_flat<false><<<grid, BLOCK, L.smem_trace + L.smem_tables, st>>>(sc, cfg, cur, hit, n_in, q, qcounts, lane_result, stats, L.n_smem_nodes, L.n_smem_tris);

@@ -59,7 +59,7 @@ constexpr int BLOCK = 256;
 constexpr int BLOCK_SHADE = 128;   // shading kernels: 128 threads x <=128 registers -> 4 blocks / SM
 
 struct Launch { int grid; size_t smem_trace, smem_tables; uint32_t n_smem_nodes, n_smem_tris; int refill_idle;
-    bool flat; int grid_flat;      // scenes of <= 32 leaves: flat traversal (kernels.cu: traverse_flat), its own grid
+    bool flat; int grid_flat;      // scenes of <= 32 leaves: flat traversal (kernels.cu: k_trace_flat), its own grid
 };
 
 // counters in the stats buffer
